@@ -26,7 +26,14 @@ Numbers in the one JSON line:
   cpu_baseline / --impl reference: the STAGED UNMODIFIED reference (oracle/_ref: vendored torch Whisper behind its own
               AlignAtt hooks) on the host cores, same per-chunk workload (oracle/ref_driver.py).
 
+--dump-outputs DIR (headline config, rank 0): what the last timed tick returned to its caller, as float32 / float64 .npy
+files -- content frames per stream, no-speech probability, token / logprob / attended frame of every decode iteration --
+and the logits its last decode left for the next one (the first streams' rows, up to 32 MB).  Weights, audio and prompts
+are seeded, so two builds run with the same arguments can be compared output for output, with a tolerance: the bf16
+path is not bit-reproducible (two runs of one build on a B200 at 1000 W: tokens identical, logits within 0.04).
+
     python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--config C] [--streams B] [--no-extras]
+                    [--dump-outputs DIR]
 Multi-GPU: python -m torch.distributed.run --nproc-per-node N bench.py --gpus N ...  (one rank per GPU; sessions are
 sharded, NCCL is used once to broadcast the packed weights; weak scaling, no data-path collective).
 """
@@ -485,7 +492,7 @@ def config_base_en_single_stream(device=0, chunks=24):
     return dict(workload="whisper base.en AlignAtt greedy, 0.5 s chunks, 1 stream, host chunk in / tokens out per call",
                 metric="ms per 0.5 s chunk (process_iter latency)", ms_p50=float(np.percentile(lat, 50)),
                 ms_p95=float(np.percentile(lat, 95)), rtf=float(lat.mean() / 1e3 / CHUNK_S),
-                mean_decode_iterations=float(np.mean(iters)), chunks=chunks)
+                mean_decode_iterations=float(np.mean(iters)), chunks=chunks, timed_steps=chunks, warmup_steps=4)
 
 
 def config_localagreement_64(device=0, streams=64, ticks=3, eng=None):
@@ -535,7 +542,8 @@ def config_localagreement_64(device=0, streams=64, ticks=3, eng=None):
     sec = float(np.mean(per))
     return dict(workload=f"whisper large-v3, LocalAgreement-shaped tick, 1.0 s chunks, {streams} ragged streams (5-15 s buffers), "
                          "32-token greedy hypothesis + word-timestamp pass per stream-tick",
-                metric=UNIT, value=streams * 1.0 / sec, ms_per_tick=sec * 1e3, rtf_per_stream=sec / 1.0, streams=streams)
+                metric=UNIT, value=streams * 1.0 / sec, ms_per_tick=sec * 1e3, rtf_per_stream=sec / 1.0, streams=streams,
+                timed_steps=ticks, warmup_steps=1)
 
 
 def config_alignatt_sortformer(device=0, streams=64, seconds=4, eng=None):
@@ -610,7 +618,7 @@ def config_alignatt_sortformer(device=0, streams=64, seconds=4, eng=None):
     return dict(workload=f"whisper large-v3 AlignAtt (0.5 s chunks, {PREFIX}+{STEPS_PER_CHUNK} tokens per chunk, full 30 s re-encode) + streaming "
                          f"Sortformer 4spk-v2 geometry (1.0 s steps, caches full: 401 rows per stream), {streams} streams per GPU, host chunks in",
                 metric=UNIT, value=streams * 1.0 / sec, ms_per_audio_second=sec * 1e3, rtf_per_stream=sec,
-                sortformer_ms_per_step=float(np.mean(diar) * 1e3), streams=streams)
+                sortformer_ms_per_step=float(np.mean(diar) * 1e3), streams=streams, timed_steps=seconds, warmup_steps=1)
 
 
 def incremental_leg(eng, scripted, B, world, rng, base, pairs=8, ticks=10, seam_bmax=0):
@@ -727,7 +735,8 @@ def config_qwen_tower(device=0, streams=128, ticks=24):
     return dict(workload=f"qwen3-asr-0.6b causal audio tower, 0.25 s chunks, raw audio in (device log-mel), {streams} streams, "
                          "host audio in / encoder rows out per call (e2e by construction)",
                 metric=UNIT, value=float(streams * 0.25 / per.mean()), ms_per_tick_mean=float(per.mean() * 1e3),
-                ms_per_tick_p95=float(np.percentile(per, 95) * 1e3), encoder_steps=int(rows), streams=streams)
+                ms_per_tick_p95=float(np.percentile(per, 95) * 1e3), encoder_steps=int(rows), streams=streams,
+                timed_steps=ticks, warmup_steps=8)
 
 
 def run_side_config(name, device):
@@ -737,6 +746,56 @@ def run_side_config(name, device):
         return fn(device)
     except Exception as e:                                                # noqa: BLE001
         return dict(error=repr(e))
+
+
+def scripted_tick(eng, sids, prefix, sup, host, last, sync_before_prefill=False):
+    """The device part of one scripted tick (module docstring) for the sessions `sids`: encode, prefill of `prefix`,
+    STEPS_PER_CHUNK greedy iterations suppressing `sup`.  Host time inside the engine calls accumulates in `host`; what
+    the tick returns to its caller goes to `last`: content frames, no-speech probabilities, and per iteration the
+    (token, logprob, attended frame) of every session."""
+    B = len(sids)
+    t0 = time.perf_counter()
+    last["content"] = eng.encode(sids)
+    t1 = time.perf_counter()
+    if sync_before_prefill:
+        eng.sync()
+        t1 = time.perf_counter()
+    eng.decode(sids, [prefix] * B)
+    t2 = time.perf_counter()
+    if sync_before_prefill:
+        host["prefill_synced"] += t2 - t1; host["ns"] += 1
+    else:
+        host["encode"] += t1 - t0; host["prefill"] += t2 - t1; host["n"] += 1
+    last["no_speech_prob"] = eng.no_speech_prob(sids)
+    last["select"] = []
+    for _ in range(STEPS_PER_CHUNK):
+        r = eng.select(sids, sup)                            # suppress -> greedy token/logprob -> alignment reduce -> frame
+        last["select"].append(r)
+        t3 = time.perf_counter()
+        eng.decode(sids, [[t[0]] for t in r])
+        if not sync_before_prefill:
+            host["step"] += time.perf_counter() - t3
+
+
+def scripted_tick_outputs(eng, sids, last, logits_bytes=32 << 20):
+    """--dump-outputs: the `last` of a tick as float arrays, and the logits its last decode left for the next iteration
+    (the first sessions' rows, up to `logits_bytes`)."""
+    sel = np.asarray(last["select"], np.float64)                           # [iteration, session, (token, logprob, frame)]
+    return dict(content_frames=np.asarray(last["content"], np.float64),
+                no_speech_prob=np.asarray(last["no_speech_prob"], np.float32),
+                tokens=sel[..., 0], logprobs=sel[..., 1].astype(np.float32), frames=sel[..., 2],
+                logits=np.stack([eng.read_logits(s) for s in sids[:max(1, logits_bytes // (4 * eng.dims.n_vocab))]]).astype(np.float32))
+
+
+def dump_outputs(out_dir, outputs, limit=64 << 20):
+    """outputs: name -> float32 / float64 array.  -> DIR/<name>.npy, at most `limit` bytes in all."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > limit:
+        raise ValueError(f"outputs of {total} bytes exceed the {limit}-byte dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -758,7 +817,13 @@ def main():
                     help="cohort: closed cohorts (best p95 capacity); continuous: arrivals join between rounds (measured: p50 0.20 s "
                          "instead of 0.34 s at 64 streams, same p95, but the small encoder batches cost capacity: 80 streams run away)")
     ap.add_argument("--seam-streams", type=int, default=0, help="first stream count probed through the seam (default: 2/3 of --streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed tick returned as DIR/<name>.npy (headline config; module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != "alignatt-large-v3" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the headline config (alignatt-large-v3) of --impl b200")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -804,7 +869,7 @@ def main():
                 return
         hib = args.config != "alignatt-base-en-1stream"
         print(json.dumps(dict(metric=r.get("metric"), value=r.get("value", r.get("ms_p50")), unit=r.get("metric"), n_gpus=world if sharded else 1,
-                              steps=args.steps, warmup=args.warmup, higher_is_better=hib, scaling="weak", vs_baseline=None,
+                              steps=r.get("timed_steps"), warmup=r.get("warmup_steps"), higher_is_better=hib, scaling="weak", vs_baseline=None,
                               dtype="bf16", data="synthetic", config=dict(workload=r.get("workload"), name=args.config),
                               e2e=dict(value=r.get("value", r.get("ms_p50")), unit=r.get("metric"),
                                        note="these configs are timed through the host-buffer API: chunk H2D and result D2H are inside"),
@@ -843,8 +908,9 @@ def main():
     rng = np.random.default_rng(1000 + rank)
     base = synthetic_audio(36.0, seed=7)
 
-    def scripted(eng, B, steps, warmup, profile_pass=True, io_only=False):
-        """The scripted tick (module docstring).  -> (ms device-resident, ms with per-chunk IO, profile, host enqueue)"""
+    def scripted(eng, B, steps, warmup, profile_pass=True, io_only=False, dump=False):
+        """The scripted tick (module docstring).  -> (ms device-resident, ms with per-chunk IO, profile, host enqueue);
+        dump: also what the last device-resident timed tick returned (module docstring, --dump-outputs)."""
         sp = eng.specials
         sids = [eng.open_session() for _ in range(B)]
         for s in sids:
@@ -854,6 +920,7 @@ def main():
         sup = sp.alignatt_suppress_tokens()
         chunk_host = torch.empty(B, CHUNK, dtype=torch.float32).pin_memory()
         host = dict(encode=0.0, prefill=0.0, prefill_synced=0.0, step=0.0, n=0, ns=0)
+        last = {}                                            # the caller-visible results of the latest tick
 
         def step(with_io, sync_before_prefill=False):
             if with_io:
@@ -862,25 +929,7 @@ def main():
                 for i, s in enumerate(sids):
                     eng.drop_audio(s, CHUNK)
                     eng.append_audio(s, cn[i])
-            t0 = time.perf_counter()
-            eng.encode(sids)
-            t1 = time.perf_counter()
-            if sync_before_prefill:
-                eng.sync()
-                t1 = time.perf_counter()
-            eng.decode(sids, [prefix] * B)
-            t2 = time.perf_counter()
-            if sync_before_prefill:
-                host["prefill_synced"] += t2 - t1; host["ns"] += 1
-            else:
-                host["encode"] += t1 - t0; host["prefill"] += t2 - t1; host["n"] += 1
-            eng.no_speech_prob(sids)
-            for _ in range(STEPS_PER_CHUNK):
-                r = eng.select(sids, sup)                    # suppress -> greedy token/logprob -> alignment reduce -> frame
-                t3 = time.perf_counter()
-                eng.decode(sids, [[t[0]] for t in r])
-                if not sync_before_prefill:
-                    host["step"] += time.perf_counter() - t3
+            scripted_tick(eng, sids, prefix, sup, host, last, sync_before_prefill)
 
         def timed(with_io, steps, warmup, profile):
             for _ in range(warmup):
@@ -929,6 +978,9 @@ def main():
             sampler.start()
         ms_dev, _ = timed(False, steps, warmup, False)
         clocks = sampler.summary() if sampler else None
+        outputs = None
+        if dump:
+            outputs = scripted_tick_outputs(eng, sids, last)
         ms_io, prof, ms_prof = None, None, None
         if profile_pass:
             ms_io, _ = timed(True, steps, max(1, warmup // 3), False)
@@ -939,7 +991,7 @@ def main():
             eng.sync()
         for s in sids:
             eng.close_session(s)
-        return dict(ms_dev=ms_dev, ms_io=ms_io, ms_prof=ms_prof, prof=prof, host=host, clocks=clocks)
+        return dict(ms_dev=ms_dev, ms_io=ms_io, ms_prof=ms_prof, prof=prof, host=host, clocks=clocks, outputs=outputs)
 
     def note(msg):
         if rank == 0:
@@ -971,7 +1023,9 @@ def main():
         return
 
     eng = make_engine(args.precision, max(B, seam_bmax), max(B, seam_bmax))
-    r = scripted(eng, B, args.steps, args.warmup)
+    r = scripted(eng, B, args.steps, args.warmup, dump=bool(args.dump_outputs) and rank == 0)
+    if r["outputs"] is not None:
+        dump_outputs(args.dump_outputs, r["outputs"])
     note(f"scripted tick: {r['ms_dev'] / args.steps:.1f} ms device-resident, {r['ms_io'] / args.steps:.1f} ms with host chunks")
     seam_best, seam_probes = None, []
     if not args.no_seam:

@@ -1,11 +1,9 @@
 """Diarization post-processing (SURVEY.md 8f-4, reference sortformer_backend.py:313-363).
-CPU: oracle/diar_oracle.py against the known answers of the reference's own tests
-(/root/reference/tests/test_sortformer_max_speakers.py:78-125, 183-215) and -- in the build container -- against the
-reference's method itself on random predictions.  GPU: the device run-length kernel (wlk_diar_segments, through the
+CPU: oracle/diar_oracle.py against the known answers of the reference's own tests (the reference project's
+tests/test_sortformer_max_speakers.py:78-125, 183-215) and against the reference's method itself on random predictions
+(recorded in tests/golden/diar_reference.npz).  GPU: the device run-length kernel (wlk_diar_segments, through the
 C ABI) against the oracle, bit-exact (integer work)."""
-import sys
-import threading
-import types
+import os
 
 import numpy as np
 import pytest
@@ -42,47 +40,16 @@ def test_oracle_speaker_cap_rules():
     assert do.process_predictions(np.zeros((0, 4), np.float32), 2, None, 0, 1.0) == ([], 0)
 
 
-def _reference_online(preds, max_speakers, len_prediction, chunk_index, gto):
-    """The reference's own method on a bare instance, NeMo stubbed out like its tests do (:18-52)."""
-    import importlib
-    import torch
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    if "soundfile" not in sys.modules:
-        m = types.ModuleType("soundfile")
-        m.__spec__ = __import__("importlib.machinery").machinery.ModuleSpec("soundfile", loader=None)
-        sys.modules["soundfile"] = m
-    for name in ("nemo", "nemo.collections", "nemo.collections.asr", "nemo.collections.asr.models", "nemo.collections.asr.modules"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules["nemo.collections.asr.models"].SortformerEncLabelModel = object
-    sys.modules["nemo.collections.asr.modules"].AudioToMelSpectrogramPreprocessor = object
-    sb = importlib.import_module("whisperlivekit.diarization.sortformer_backend")
-    online = object.__new__(sb.SortformerDiarizationOnline)
-    online.total_preds = torch.tensor(np.asarray(preds)[None], dtype=torch.float32)
-    online.max_speakers = max_speakers
-    online._len_prediction = len_prediction
-    online.chunk_duration_seconds = 0.96
-    online.segment_lock = threading.Lock()
-    online._chunk_index = chunk_index
-    online.global_time_offset = gto
-    return [(int(s.speaker), s.start, s.end) for s in online._process_predictions()], online._len_prediction
-
-
-@pytest.mark.reference
 def test_oracle_equals_reference_method_on_random_predictions():
-    rng = np.random.default_rng(5)
-    for trial in range(40):
-        n_spk = 4
-        T = int(rng.integers(1, 60))
-        preds = rng.random((T, n_spk)).astype(np.float32)
-        if trial % 3 == 0:                                              # long runs + exact ties
-            preds = np.repeat(np.round(preds[: max(1, T // 4)], 1), 4, axis=0)[:T]
-        cap = int(rng.integers(1, 5))
-        lp = None if trial % 2 == 0 else int(rng.integers(1, T + 1))
-        chunk, gto = int(rng.integers(0, 50)), float(rng.choice([0.0, 1.37, 12.5]))
-        ref, ref_lp = _reference_online(preds, cap, lp, chunk, gto)
+    """The reference's _process_predictions on seeded random cases, recorded by oracle/make_golden_seams.py."""
+    from oracle.make_golden_seams import diar_cases
+    g = dict(np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "diar_reference.npz")))
+    off = g["offsets"]
+    for trial, (preds, cap, lp, chunk, gto) in enumerate(diar_cases()):
+        sl = slice(off[trial], off[trial + 1])
+        ref = [(int(s), float(a), float(b)) for s, a, b in zip(g["speaker"][sl], g["start"][sl], g["end"][sl])]
         mine, my_lp = do.process_predictions(preds, cap, lp, chunk, 0.96, gto)
-        assert (mine, my_lp) == (ref, ref_lp), trial
+        assert (mine, my_lp) == (ref, int(g["len_prediction"][trial])), trial
 
 
 # ------------------------------------------------------------------------------------------ GPU

@@ -1,10 +1,7 @@
-"""Build container only: the LocalAgreement seam.  The reference's unchanged whisper.transcribe()
-(DecodingTask, temperature fallback, timestamp rules, find_alignment + DTW) runs over
+"""Needs the reference package staged under oracle/_ref by build(): the LocalAgreement seam.  The reference's
+unchanged whisper.transcribe() (DecodingTask, temperature fallback, timestamp rules, find_alignment + DTW) runs over
 B200TranscribeModel; with the CPU oracle behind the engine API the result must equal what the same
 transcribe() produces over the reference's own torch Whisper on the same weights and audio."""
-import sys
-import types
-
 import numpy as np
 import pytest
 import torch
@@ -15,18 +12,11 @@ pytestmark = pytest.mark.reference
 
 
 def _import_reference():
-    if "soundfile" not in sys.modules:
-        m = types.ModuleType("soundfile")
-        m.__spec__ = __import__("importlib.machinery").machinery.ModuleSpec("soundfile", loader=None)   # find_spec() must not choke on the stub
-        m.read = m.write = m.info = lambda *a, **k: (_ for _ in ()).throw(RuntimeError("stub"))
-        sys.modules["soundfile"] = m
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import whisperlivekit  # noqa: F401
+    from oracle import stage_reference
+    stage_reference.import_staged_reference()
 
 
 def _ref_model(dims, sd, heads):
-    sys.path.insert(0, "/root/repo/oracle")
     from oracle.make_golden import build_reference_model
     return build_reference_model(dims, sd, heads)
 

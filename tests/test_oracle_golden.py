@@ -80,13 +80,11 @@ def test_alignment_heads_table_shape():
         assert heads == sorted(heads)
 
 
-@pytest.mark.reference
 def test_alignment_heads_match_reference():
-    import base64, gzip, re, ast
-    src = open("/root/reference/whisperlivekit/whisper/__init__.py").read()
-    dumps = ast.literal_eval(re.search(r"_ALIGNMENT_HEADS = (\{.*?\n\})", src, re.S).group(1))
+    """The reference's _ALIGNMENT_HEADS table, decoded (oracle/make_golden_seams.py)."""
+    g = load_case("alignment_heads")
     for k, heads in ALIGNMENT_HEADS.items():
         d = DIMS[k]
-        a = np.frombuffer(gzip.decompress(base64.b85decode(dumps[k])), dtype=bool)
-        a = a.reshape(d.n_text_layer, d.n_text_head)
+        a = g[k]
+        assert a.shape == (d.n_text_layer, d.n_text_head)
         assert [(int(l), int(h)) for l, h in zip(*np.nonzero(a))] == heads

@@ -1,5 +1,6 @@
 """CPU: the Silero VAD oracle against probabilities recorded from the reference's scripted model
-(oracle/make_golden_vad.py): seeded weights everywhere; with the trained weights only where /root/reference exists."""
+(oracle/make_golden_vad.py): seeded weights everywhere; with the trained weights where build() staged the reference
+package under oracle/_ref."""
 import os
 
 import numpy as np
@@ -27,9 +28,10 @@ def test_vad_oracle_matches_reference_model_with_seeded_weights():
 @pytest.mark.reference
 def test_vad_oracle_matches_reference_model_with_trained_weights():
     import torch
+    from oracle.stage_reference import TARGET
     from oracle.vad_oracle import VadOracle
     g = dict(np.load(os.path.join(HERE, "golden", "vad.npz")))
-    m = torch.jit.load("/root/reference/whisperlivekit/silero_vad_models/silero_vad.jit", map_location="cpu")
+    m = torch.jit.load(os.path.join(TARGET, "whisperlivekit", "silero_vad_models", "silero_vad.jit"), map_location="cpu")
     o = VadOracle({k: v.numpy() for k, v in m.state_dict().items()})
     audio, n = _audio(), int(g["n_windows"])
     a, b = o.open_session(), o.open_session()

@@ -1,10 +1,9 @@
-"""Build container only (needs /root/reference): ``plugin.install()`` executed against the reference's own
-``SimulStreamingASR`` / ``SimulStreamingOnlineProcessor`` (simul_whisper/backend.py:61-71, 530-553), and the two hooks
-no other test reaches -- ``lang_id`` (simul_whisper.py:266-292) and the CIF end-of-word test
+"""Needs the reference package staged under oracle/_ref by build(): ``plugin.install()`` executed against the
+reference's own ``SimulStreamingASR`` / ``SimulStreamingOnlineProcessor`` (simul_whisper/backend.py:61-71, 530-553),
+and the two hooks no other test reaches -- ``lang_id`` (simul_whisper.py:266-292) and the CIF end-of-word test
 (eow_detection.py:37-77).  The CUDA engine is replaced by the CPU oracle through ``install(engine_factory=...)``:
 what is under test is the registration and the hooks, not the kernels (those are the -m gpu tests)."""
 import os
-import sys
 import types
 
 import numpy as np
@@ -13,18 +12,16 @@ import torch
 
 from golden_util import case_setup
 
-pytestmark = pytest.mark.reference
+
+@pytest.fixture(autouse=True)
+def _reference_on_the_cpu(monkeypatch):
+    """The reference puts AlignAtt on the GPU whenever one is visible; here it runs next to the CPU oracle."""
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
 
 
 def _import_reference():
-    if "soundfile" not in sys.modules:
-        m = types.ModuleType("soundfile")
-        m.__spec__ = __import__("importlib.machinery").machinery.ModuleSpec("soundfile", loader=None)
-        m.read = m.write = m.info = lambda *a, **k: (_ for _ in ()).throw(RuntimeError("stub"))
-        sys.modules["soundfile"] = m
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import whisperlivekit  # noqa: F401
+    from oracle import stage_reference
+    stage_reference.import_staged_reference()
 
 
 ASR_KW = dict(decoder_type="greedy", beams=1, model_size=None, model_path=None, decoder_model_path=None,
@@ -44,6 +41,7 @@ def _checkpoint(tmp_path, name, dims, sd, heads):
     return path
 
 
+@pytest.mark.reference
 def test_install_routes_simulstreaming_through_the_engine(tmp_path, monkeypatch):
     _import_reference()
     import whisperlivekit.simul_whisper.backend as be
@@ -107,6 +105,7 @@ def test_install_routes_simulstreaming_through_the_engine(tmp_path, monkeypatch)
     assert toks_b200 == toks_ref
 
 
+@pytest.mark.reference
 def test_lang_id_hook_matches_reference():
     _import_reference()
     from oracle import whisper_oracle as wo
@@ -142,6 +141,7 @@ def test_lang_id_hook_matches_reference():
     assert isinstance(ours.infer(is_last=False), list)
 
 
+@pytest.mark.reference
 def test_cif_fire_at_boundary_matches_reference(tmp_path):
     _import_reference()
     from oracle import whisper_oracle as wo
@@ -178,6 +178,30 @@ def test_cif_fire_at_boundary_matches_reference(tmp_path):
         fired.append(f_r)
     # and through the whole infer(): the CIF decision only changes how many tokens are kept (align_att_base.py:296)
     assert isinstance(ours.infer(is_last=False), list)
+
+
+@pytest.mark.reference
+def test_reference_diarization_factory_builds_the_sortformer_drop_in():
+    """plugin.install_sortformer() + the reference's unchanged core.online_diarization_factory (core.py:468-480): its own
+    import statement resolves to the B200 drop-in and its calling convention constructs it.  The shared model carries
+    only what that constructor reads; the drop-ins run end to end on the GPU in
+    tests/test_gpu_sortformer.py::test_registration_as_the_reference_backend_module."""
+    _import_reference()
+    from whisperlivekit_b200 import plugin
+    from whisperlivekit_b200.sortformer_dims import SORTFORMER_DIMS
+    from whisperlivekit_b200.sortformer_engine import B200SortformerDiarizationOnline
+    d = SORTFORMER_DIMS["small"]
+    mod = plugin.install_sortformer(dims=d)
+    try:
+        from whisperlivekit.core import online_diarization_factory
+        opened = []
+        engine = types.SimpleNamespace(chunk_duration_seconds=1.0, device=0, open_session=lambda: opened.append(7) or 7)
+        args = types.SimpleNamespace(diarization_backend="sortformer", sortformer_max_speakers=2)
+        online = online_diarization_factory(args, types.SimpleNamespace(engine=engine, dims=d))
+        assert type(online) is mod.SortformerDiarizationOnline is B200SortformerDiarizationOnline
+        assert online.engine is engine and online.sid == 7 and opened == [7] and online.max_speakers == 2
+    finally:
+        plugin.uninstall_sortformer()
 
 
 def test_nemo_checkpoint_reader_needs_no_nemo(tmp_path):

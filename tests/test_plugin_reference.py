@@ -1,10 +1,7 @@
-"""Build container only (needs /root/reference): the drop-in seam.  The reference's own
+"""Needs the reference package staged under oracle/_ref by build(): the drop-in seam.  The reference's own
 AlignAttBase.infer() drives our hooks (AlignAttHooks); with the CPU oracle standing in for the
 CUDA engine behind the same session API, the emitted tokens / attended frames must equal what the
 reference's AlignAtt produced (the golden fixtures)."""
-import sys
-import types
-
 import numpy as np
 import pytest
 import torch
@@ -14,15 +11,15 @@ from golden_util import case_setup
 pytestmark = pytest.mark.reference
 
 
+@pytest.fixture(autouse=True)
+def _reference_on_the_cpu(monkeypatch):
+    """The reference puts AlignAtt on the GPU whenever one is visible; here it runs next to the CPU oracle."""
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
+
+
 def _import_reference():
-    if "soundfile" not in sys.modules:
-        m = types.ModuleType("soundfile")
-        m.__spec__ = __import__("importlib.machinery").machinery.ModuleSpec("soundfile", loader=None)   # find_spec() must not choke on the stub
-        m.read = m.write = m.info = lambda *a, **k: (_ for _ in ()).throw(RuntimeError("stub"))
-        sys.modules["soundfile"] = m
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import whisperlivekit  # noqa: F401
+    from oracle import stage_reference
+    stage_reference.import_staged_reference()
 
 
 @pytest.mark.parametrize("name", ["micro", "microml"])
