@@ -172,11 +172,25 @@ int wlk_read_align_attn(wlk_engine* e, int32_t sid, float* out, int64_t capacity
  *      backend: WLK_BACKEND_SIMT, WLK_BACKEND_TCGEN05 (auto tile choice), 3 = force the one-CTA tcgen05 kernel,
  *      4 = force the CTA-pair (cta_group::2) kernel.
  *      a_type/w_type/c_type: 0 = fp32, 1 = bf16.  C[M,N] = act(A[M,K] W[N,K]^T + bias); `gelu` is a flag
- *      word: bit 0 = erf-GELU, bit 1 = accumulate into the fp32 C in place (C += A W^T + bias).           */
+ *      word: bit 0 = erf-GELU, bit 1 = accumulate into the fp32 C in place (C += A W^T + bias).
+ *      w_type 2 = the WLK_PREC_BF16X3 split operands (tcgen05 backends only): W is the bf16 hi plane, the lo plane
+ *      sits right behind it at W + N * ldw; A is fp32 and is split on the fly.                                */
 int wlk_op_gemm(wlk_engine* e, int backend, const void* A, int a_type, int64_t lda,
                 const void* W, int w_type, int64_t ldw, const float* bias,
                 void* C, int c_type, int64_t ldc, int M, int N, int K, int gelu);
+/* encoder self-attention over qkv [batch * 1500, 3 * n_audio_state] (q, k pre-scaled by 64^-0.25) -> out
+ * [batch * 1500, n_audio_state].  backend 3 = force the one-query-tile tcgen05 kernel.  type 0 = fp32, 1 = bf16,
+ * 2 = split planes (tcgen05): qkv is the bf16 hi plane with the lo plane right behind it, out is fp32.             */
 int wlk_op_encoder_attention(wlk_engine* e, int backend, const void* qkv, int type, int batch, void* out);
+/* One decoder layer's attention over caches the caller owns, with the dispatch wlk_decode runs (backend
+ * WLK_BACKEND_SIMT or WLK_BACKEND_TCGEN05 = the bf16 prefill kernels; type 0 = fp32, 1 = bf16).
+ *   kind 0: causal self-attention, kv[i] = [n_text_layer][2][n_text_head][n_text_ctx][64];
+ *   kind 1: cross-attention, kv[i] = [n_text_layer][2][n_text_head][1500][64]; the softmaxed rows of the engine's
+ *           alignment heads go to align[i] = [n_align][n_text_ctx][1500] fp32 from row align_row0[i] on.
+ * q and out are [sum n_rows][n_text_state], packed by job; row t of job i is at position offsets[i] + t.           */
+int wlk_op_decoder_attention(wlk_engine* e, int kind, int backend, int type, int layer, const void* q, int n_jobs,
+                             const int32_t* n_rows, const int32_t* offsets, const int32_t* align_row0,
+                             const void* const* kv, float* const* align, void* out);
 
 /* ---- word-timestamp kernels of the LocalAgreement path: native replacements of the reference's Triton
  *      median_kernel / dtw_kernel (whisper/triton_ops.py:13-103) with the semantics of its CPU path

@@ -187,3 +187,166 @@ def test_gemm_tcgen05_split_k_in_place(eng, M, N, K):
     eng.sync()
     ref = x0 + A.float() @ W.float().t() + b
     assert (x - ref).abs().max().item() < 1e-3 * max(1.0, ref.abs().max().item())
+
+
+# ---- one-query-tile encoder attention and the split-operand (bf16x3) kernels, against fp64 -----------------------------
+def _enc_engine(d, H):
+    from whisperlivekit_b200.dims import ModelDimensions
+    from whisperlivekit_b200.engine import WhisperEngine
+    return WhisperEngine(ModelDimensions(80, 1500, d, H, 1, 51864, 448, 64, 1, 1), None, [(0, 0)], precision="bf16",
+                         max_sessions=1, max_batch=1)
+
+
+def _enc_ref64(qkv, B, H):
+    """fp64 softmax(Q K^T) V of the fused [B*1500, 3d] buffer -> (out [B*1500, d], scores [B, H, 1500, 1500])."""
+    x = qkv.double().view(B, 1500, 3, H, 64)
+    q, k, v = x[:, :, 0].transpose(1, 2), x[:, :, 1].transpose(1, 2), x[:, :, 2].transpose(1, 2)
+    s = q @ k.transpose(-1, -2)
+    return (torch.softmax(s, dim=-1) @ v).transpose(1, 2).reshape(B * 1500, H * 64), s
+
+
+def _enc_run(e, backend, qkv, code, B, d):
+    out = torch.full((B * 1500, d), float("nan"), device="cuda", dtype=torch.float32 if code != 1 else torch.bfloat16)
+    torch.cuda.synchronize()
+    e.op_encoder_attention(backend, qkv.data_ptr(), code, B, out.data_ptr())
+    e.sync()
+    return out.double()
+
+
+def _enc_inputs(B, H, seed, ramp):
+    """fp32 q|k|v [B*1500, 3d] of std 0.7-0.8; ramp: key norms grow tile by tile (and shrink on one head), as in
+    test_encoder_attention_tcgen05_moving_reference, so that most rows move their softmax reference."""
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    if not ramp:
+        return torch.randn(B * 1500, 3 * H * 64, device="cuda", generator=g) * 0.8
+    x = torch.randn(B, 1500, 3, H, 64, device="cuda", generator=g) * 0.7
+    r = torch.ones(1500, device="cuda")
+    r[400:] = 1.8; r[700:] = 2.6; r[1000:] = 3.5; r[1300:] = 4.5
+    x[:, :, 1] *= r[None, :, None, None]
+    x[1 % B, :, 1, 1] *= torch.linspace(1.0, 0.2, 1500, device="cuda")[:, None]
+    return x.reshape(B * 1500, 3 * H * 64)
+
+
+def _moving_share(s):
+    jump = (s[..., 1280:].amax(-1) - s[..., :128].amax(-1)) * 1.4427                # log2 units, last tile vs first
+    return (jump > 8).double().mean().item()
+
+
+@pytest.mark.parametrize("d,H,B", [(128, 2, 1), (384, 6, 2), (1280, 20, 1)])
+def test_encoder_attention_tcgen05_one_tile(d, H, B):
+    """The one-query-tile kernel (backend 3: the kernel body of the decoder prefills and of the bf16x3 mode; the
+    encoder's default is the two-tile kernel) vs fp64 on the same bf16 inputs: 2e-2 on O(1) outputs (P in bf16).
+    Measured on a B200 (1000 W): 1.3e-2 to 1.4e-2."""
+    e2 = _enc_engine(d, H)
+    qkv = _enc_inputs(B, H, d + 1, ramp=False).bfloat16()
+    out = _enc_run(e2, "tcgen05_1tile", qkv, 1, B, d)
+    ref, _ = _enc_ref64(qkv, B, H)
+    assert not torch.isnan(out).any()
+    err = (out - ref).abs().max().item()
+    print(f"one-tile encoder attention d={d} B={B}: max err {err:.3e}")
+    assert err < 2e-2
+    e2.close()
+
+
+def test_encoder_attention_tcgen05_one_tile_moving_reference():
+    """The one-tile kernel on inputs where most rows move their softmax reference (rescale of O and l in TMEM).
+    Measured on a B200 (1000 W): 1.4e-2."""
+    d, H, B = 256, 4, 2
+    e2 = _enc_engine(d, H)
+    qkv = _enc_inputs(B, H, 77, ramp=True).bfloat16()
+    out = _enc_run(e2, "tcgen05_1tile", qkv, 1, B, d)
+    ref, s = _enc_ref64(qkv, B, H)
+    assert _moving_share(s) > 0.5                                                    # the path under test is taken
+    assert not torch.isnan(out).any()
+    err = (out - ref).abs().max().item()
+    print(f"one-tile encoder attention, moving reference: max err {err:.3e}")
+    assert err < 2e-2
+    e2.close()
+
+
+@pytest.mark.parametrize("ramp", [False, True], ids=["random", "moving_reference"])
+def test_encoder_attention_bf16x3(ramp):
+    """Split-plane attention (type 2: bf16 hi plane with the lo plane behind it, fp32 out) vs fp64 on the raw fp32
+    inputs: within 1e-3, and at most 1/10 of the one-tile bf16 kernel's error on the same inputs -- Q K^T and P V
+    each take three MMAs (hi hi + lo hi + hi lo), so every dropped lo term shows.  Measured on a B200 (1000 W):
+    1.0e-4 (random) and 2.8e-4 (ramp) against 5.3e-2 and 1.4e-1 for the bf16 kernel."""
+    d, H, B = 384, 6, 2
+    e2 = _enc_engine(d, H)
+    x = _enc_inputs(B, H, 91, ramp)
+    hi = x.bfloat16()
+    planes = torch.cat([hi, (x - hi.float()).bfloat16()])
+    ref, s = _enc_ref64(x, B, H)
+    if ramp:
+        assert _moving_share(s) > 0.5
+    out = _enc_run(e2, "tcgen05", planes, 2, B, d)
+    err = (out - ref).abs().max().item()
+    err_bf16 = (_enc_run(e2, "tcgen05_1tile", hi, 1, B, d) - ref).abs().max().item()
+    print(f"bf16x3 encoder attention ({'ramp' if ramp else 'random'}): max err {err:.3e}, bf16 one-tile {err_bf16:.3e}")
+    assert not torch.isnan(out).any()
+    assert err < 1e-3 and err < err_bf16 / 10, (err, err_bf16)
+    e2.close()
+
+
+def _x3_check(eng, backend, A, A_bf, W, b, in_place=False):
+    """bf16x3 GEMM (w_type 2: W's hi plane, the lo plane right behind it; fp32 A split on the fly) vs fp64 on the fp32
+    operands: |err| <= 2e-4 max(1, |ref|) elementwise (~16 mantissa bits per product), and at most 1/20 of the plain
+    bf16 kernel's error on the same operands, which only holds when both lo-plane MMAs contribute.  Measured on a B200
+    (1000 W): at most 3.5e-5, against 9e-3 to 1.3e-2 for the bf16 kernel."""
+    M, K = A.shape
+    N = W.shape[0]
+    g = torch.Generator(device="cuda").manual_seed(M + N)
+    x0 = torch.randn(M, N, device="cuda", generator=g) if in_place else torch.zeros(M, N, device="cuda")
+    ref = x0.double() + A.double() @ W.double().t() + b.double()
+    W_hi = W.bfloat16()
+    planes = torch.cat([W_hi, (W - W_hi.float()).bfloat16()])
+    flags = 2 if in_place else 0
+    out3, outb = x0.clone(), x0.clone()
+    torch.cuda.synchronize()
+    eng.op_gemm(backend, A.data_ptr(), 0, A.stride(0), planes.data_ptr(), 2, K, b.data_ptr(), out3.data_ptr(), 0, N,
+                M, N, K, flags)
+    eng.op_gemm(backend, A_bf.data_ptr(), 1, A_bf.stride(0), W_hi.data_ptr(), 1, K, b.data_ptr(), outb.data_ptr(), 0, N,
+                M, N, K, flags)
+    eng.sync()
+    err3 = (out3.double() - ref).abs()
+    errb = (outb.double() - ref).abs().max().item()
+    print(f"bf16x3 gemm {backend} {M}x{N}x{K}{' in place' if in_place else ''}: max err {err3.max().item():.3e}, "
+          f"bf16 {errb:.3e}")
+    assert torch.all(err3 <= 2e-4 * ref.abs().clamp(min=1.0)), err3.max().item()
+    assert err3.max().item() <= errb / 20, (err3.max().item(), errb)
+
+
+X3_SHAPES = [("tcgen05", 16, 1280, 5120), ("tcgen05", 129, 264, 72), ("tcgen05", 1500, 1280, 1280),
+             ("tcgen05", 3000, 5120, 1280), ("tcgen05_1cta", 1500, 1280, 1280), ("tcgen05_1cta", 129, 264, 72),
+             ("tcgen05_1cta", 64, 1280, 5120), ("tcgen05_pair", 512, 512, 256), ("tcgen05_pair", 257, 300, 72),
+             ("tcgen05_pair", 1000, 3840, 1280)]
+
+
+@pytest.mark.parametrize("backend,M,N,K", X3_SHAPES)
+def test_gemm_bf16x3(eng, backend, M, N, K):
+    """Auto tiles (split-K for 16 x 1280 x 5120, the CTA pair for 3000 x 5120), the one-CTA and the CTA-pair kernel."""
+    g = torch.Generator(device="cuda").manual_seed(M * 3 + N + K)
+    A = torch.randn(M, K, device="cuda", generator=g)
+    W = torch.randn(N, K, device="cuda", generator=g) / K ** 0.5
+    b = torch.randn(N, device="cuda", generator=g)
+    _x3_check(eng, backend, A, A.bfloat16(), W, b)
+
+
+@pytest.mark.parametrize("M,N,K", [(16, 1280, 1280), (64, 1280, 5120), (48, 512, 512)])
+def test_gemm_bf16x3_in_place(eng, M, N, K):
+    """x += A W^T + b on the fp32 residual stream, as the bf16x3 decoder runs it (split-K with fp32 atomics for K 5120)."""
+    g = torch.Generator(device="cuda").manual_seed(M + N + K + 1)
+    A = torch.randn(M, K, device="cuda", generator=g)
+    W = torch.randn(N, K, device="cuda", generator=g) / K ** 0.5
+    b = torch.randn(N, device="cuda", generator=g)
+    _x3_check(eng, "tcgen05", A, A.bfloat16(), W, b, in_place=True)
+
+
+def test_gemm_bf16x3_strided_overlapping_rows(eng):
+    """The conv stem's view with overlapping rows (lda 80 < K 240): the split covers the whole underlying range."""
+    g = torch.Generator(device="cuda").manual_seed(6)
+    base = torch.randn(3002 * 80, device="cuda", generator=g)
+    A = torch.as_strided(base, (3000, 240), (80, 1))
+    A_bf = torch.as_strided(base.bfloat16(), (3000, 240), (80, 1))
+    W = torch.randn(384, 240, device="cuda", generator=g) / 15
+    b = torch.randn(384, device="cuda", generator=g)
+    _x3_check(eng, "tcgen05", A, A_bf, W, b)

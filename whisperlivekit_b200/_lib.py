@@ -125,6 +125,8 @@ SIGNATURES = {
     "wlk_op_gemm": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_int64, _vp, C.c_int, C.c_int64, _vp,
                               _vp, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int]),
     "wlk_op_encoder_attention": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_int, _vp]),
+    "wlk_op_decoder_attention": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp,
+                                           _vp, _vp]),
     "wlk_op_encoder_attention_trace": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp]),
     "wlk_op_median_filter": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int]),
     "wlk_op_dtw": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp, _vp, _i32p]),

@@ -430,6 +430,11 @@ void enc_attention_tcgen05(const void* qkv, int batch, int n_head, int d_model, 
     // one-tile CTA, which also serves the decoder prefills and the split-operand mode
     static const bool two_tile = [] { const char* v = getenv("WLK_ATTN2"); return !(v && v[0] == '0'); }();
     if (two_tile && trace_dev == nullptr) { enc_attention_tcgen05_two_tile(qkv, batch, n_head, d_model, out, st); return; }
+    enc_attention_tcgen05_one_tile(qkv, batch, n_head, d_model, out, st, trace_dev);
+}
+
+void enc_attention_tcgen05_one_tile(const void* qkv, int batch, int n_head, int d_model, void* out, cudaStream_t st,
+                                    long long* trace_dev) {
     CUtensorMap tm;
     std::string err;
     WLK_CHECK(make_tmap_bf16_2d(&tm, qkv, (uint64_t)batch * N_CTX, (uint64_t)3 * d_model, (uint64_t)3 * d_model, BQ, DH, &err),

@@ -822,6 +822,32 @@ void encode_incremental(wlk_engine* e, const int32_t* sids, int n, int32_t* cont
 }
 
 // ---------------------------------------------------------------------------------------
+// decoder attention of one layer over the jobs' caches (decode_batch and wlk_op_decoder_attention): `q` / `out` are
+// the packed rows [R][n_text_state] of `type`, max_rows the largest n_rows of a job.  tensor_cores: the bf16 tcgen05
+// prefill kernels, which read the caches through the tensor maps at maps_dev[job.slot].
+// ---------------------------------------------------------------------------------------
+void dec_self_attention_layer(wlk_engine* e, const void* q, int type, int R, const DecJob* jobs_dev, int n, int max_rows,
+                              int layer, const void* self_maps_dev, void* out, bool tensor_cores) {
+    const wlk_dims& D = e->dims;
+    // prefills on the tensor cores (causal, per-session cache planes through TMA); token steps and the fp32 modes on
+    // the SIMT kernel
+    if (tensor_cores)
+        dec_self_attention_tcgen05(q, R, jobs_dev, n, max_rows, layer, D.n_text_head, D.n_text_state, D.n_text_ctx,
+                                   self_maps_dev, out, e->st);
+    else
+        dec_self_attention(q, type, jobs_dev, n, layer, D.n_text_head, D.n_text_state, D.n_text_ctx, out, max_rows, e->st);
+}
+void dec_cross_attention_layer(wlk_engine* e, const void* q, int type, int R, const DecJob* jobs_dev, int n, int max_rows,
+                               int layer, const void* cross_maps_dev, void* out, bool tensor_cores) {
+    const wlk_dims& D = e->dims;
+    if (tensor_cores)     // all non-alignment heads on the tensor cores; alignment heads need the exported rows
+        dec_cross_attention_tcgen05(q, R, jobs_dev, n, max_rows, layer, D.n_text_head, D.n_text_state, cross_maps_dev,
+                                    e->align_rank_dev, out, e->st);
+    dec_cross_attention(q, type, jobs_dev, n, layer, D.n_text_head, D.n_text_state, D.n_text_ctx, e->align_rank_dev, out,
+                        max_rows, tensor_cores, e->st);
+}
+
+// ---------------------------------------------------------------------------------------
 // decode: one TextDecoder.forward over packed rows of several sessions
 // ---------------------------------------------------------------------------------------
 void decode_batch(wlk_engine* e, const int32_t* sids, int n, const int32_t* tokens, const int32_t* offsets,
@@ -869,6 +895,7 @@ void decode_batch(wlk_engine* e, const int32_t* sids, int n, const int32_t* toke
     }
     sg.upload();
 
+    const bool tc_prefill = e->attn_backend == WLK_BACKEND_TCGEN05 && e->act == DT_BF16 && max_tq >= 16;
     auto launch_all = [&]() {
     {   ProfScope ps(e, WLK_KC_MISC);
         embed_tokens(tok_dev, pos_dev, W.emb_f32, W.dec_pos, e->dx, R, dt, e->st); }
@@ -886,12 +913,7 @@ void decode_batch(wlk_engine* e, const int32_t* sids, int n, const int32_t* toke
             g.epi.layer = li; g.epi.n_head = H; g.epi.d_model = dt; g.epi.kv_len = ctx;
             run_gemm(e, g, WLK_KC_GEMM_DEC); }
         {   ProfScope ps(e, WLK_KC_ATTN_DEC_SELF);
-            // prefills on the tensor cores (causal, per-session cache planes through TMA); token steps and the fp32
-            // modes on the SIMT kernel
-            if (e->attn_backend == WLK_BACKEND_TCGEN05 && e->act == DT_BF16 && max_tq >= 16)
-                dec_self_attention_tcgen05(e->dq, R, dj_dev, n, max_tq, li, H, dt, ctx, e->self_maps_dev, e->datt, e->st);
-            else
-                dec_self_attention(e->dq, e->act, dj_dev, n, li, H, dt, ctx, e->datt, max_tq, e->st); }
+            dec_self_attention_layer(e, e->dq, e->act, R, dj_dev, n, max_tq, li, e->self_maps_dev, e->datt, tc_prefill); }
         {   GemmArgs g;
             g.A = e->datt; g.a_type = e->act; g.lda = dt; g.W = L.Wo; g.w_type = e->wt; g.ldw = dt;
             g.M = R; g.N = dt; g.K = dt;
@@ -906,11 +928,7 @@ void decode_batch(wlk_engine* e, const int32_t* sids, int n, const int32_t* toke
             g.epi.C = e->dq; g.epi.c_type = e->act; g.epi.ldc = dt;
             run_gemm(e, g, WLK_KC_GEMM_DEC); }
         {   ProfScope ps(e, WLK_KC_ATTN_DEC_CROSS, 0, (double)n * 2 * H * N_CTX * 64 * es);
-            const bool tc_prefill = e->attn_backend == WLK_BACKEND_TCGEN05 && e->act == DT_BF16 && max_tq >= 16;
-            if (tc_prefill)     // all non-alignment heads on the tensor cores; alignment heads need the exported rows
-                dec_cross_attention_tcgen05(e->dq, R, dj_dev, n, max_tq, li, H, dt, e->kv_maps_dev, e->align_rank_dev,
-                                            e->datt, e->st);
-            dec_cross_attention(e->dq, e->act, dj_dev, n, li, H, dt, ctx, e->align_rank_dev, e->datt, max_tq, tc_prefill, e->st); }
+            dec_cross_attention_layer(e, e->dq, e->act, R, dj_dev, n, max_tq, li, e->kv_maps_dev, e->datt, tc_prefill); }
         {   GemmArgs g;
             g.A = e->datt; g.a_type = e->act; g.lda = dt; g.W = L.Woc; g.w_type = e->wt; g.ldw = dt;
             g.M = R; g.N = dt; g.K = dt;
@@ -1234,6 +1252,22 @@ float* tap_buffer(wlk_engine* e, size_t n) {
     }
     return e->tap_host;
 }
+
+// per-call device memory of an op-level entry point: freed once the engine's stream has drained (also when the call
+// fails half-way)
+struct CallBuffers {
+    wlk_engine* e;
+    std::vector<void*> bufs;
+    explicit CallBuffers(wlk_engine* e_) : e(e_) {}
+    void* take(size_t bytes) { bufs.push_back(dmalloc_bytes(bytes, nullptr)); return bufs.back(); }
+    ~CallBuffers() {
+        if (bufs.empty()) return;
+        cudaStreamSynchronize(e->st);
+        for (void* p : bufs) cudaFree(p);
+    }
+};
+
+bool aligned16(const void* p) { return p != nullptr && reinterpret_cast<uintptr_t>(p) % 16 == 0; }
 
 }  // namespace
 }  // namespace wlk
@@ -1785,12 +1819,27 @@ int wlk_op_gemm(wlk_engine* e, int backend, const void* A, int a_type, int64_t l
                 const float* bias, void* C, int c_type, int64_t ldc, int M, int N, int K, int gelu) {
     WLK_API_BEGIN
     LOCK(e);
+    WLK_CHECK(A && Wm && C, "null argument");
+    WLK_CHECK(M >= 1 && N >= 1 && K >= 1, "empty problem %d x %d x %d", M, N, K);
+    CallBuffers cb(e);
     GemmArgs g;
     g.A = A; g.a_type = a_type; g.lda = lda; g.W = Wm; g.w_type = w_type; g.ldw = ldw; g.M = M; g.N = N; g.K = K;
     g.epi.bias = bias; g.epi.gelu = gelu & 1; g.epi.C = C; g.epi.c_type = c_type; g.epi.ldc = ldc;
     g.sk_scratch = e->sk_scratch; g.sk_scratch_floats = SK_SCRATCH_FLOATS;
     g.sk_counters = e->sk_counters; g.sk_max_tiles = SK_MAX_TILES;
     if (gelu & 2) { WLK_CHECK(c_type == DT_F32, "in-place accumulation needs an fp32 output"); g.epi.residual = (const float*)C; g.epi.ldr = ldc; }
+    if (w_type == DT_BF16X2) {
+        // split operands (the bf16x3 mode): W is the hi plane with the lo plane right behind it, as run_gemm lays out
+        // the weights; the fp32 A is split into (hi, lo) planes over its whole range (M - 1) lda + K (overlapping
+        // conv views included), in the engine's scratch when it is large enough, else in per-call memory
+        WLK_CHECK(backend == WLK_BACKEND_TCGEN05 || backend == 3 || backend == 4,
+                  "the bf16x3 GEMM runs on the tensor cores only (backend 2, 3 or 4)");
+        WLK_CHECK(lda >= 1 && ldw >= K, "bad row pitch");
+        g.W_lo = reinterpret_cast<const bf16*>(Wm) + (size_t)N * ldw;
+        const size_t need = ((size_t)(M - 1) * lda + K + 7) / 8 * 8;   // whole 16-byte units: the lo plane stays aligned
+        if (e->a_split && need <= e->a_split_elems) { g.a_split = e->a_split; g.a_split_elems = e->a_split_elems; }
+        else { g.a_split = cb.take(need * 2 * sizeof(bf16)); g.a_split_elems = need; }
+    }
     ProfScope ps(e, WLK_KC_MISC, 2.0 * M * (double)N * K, 0);
     if (backend == WLK_BACKEND_TCGEN05) gemm_tcgen05(g, e->st, e->num_sms, 0);
     else if (backend == 3) gemm_tcgen05(g, e->st, e->num_sms, 1);
@@ -1801,13 +1850,85 @@ int wlk_op_gemm(wlk_engine* e, int backend, const void* A, int a_type, int64_t l
 int wlk_op_encoder_attention(wlk_engine* e, int backend, const void* qkv, int type, int batch, void* out) {
     WLK_API_BEGIN
     LOCK(e);
-    ProfScope ps(e, WLK_KC_MISC, 4.0 * batch * e->dims.n_audio_head * (double)N_CTX * N_CTX * 64, 0);
-    if (backend == WLK_BACKEND_TCGEN05) {
+    WLK_CHECK(aligned16(qkv) && aligned16(out), "qkv and out must be non-null and 16-byte aligned");
+    WLK_CHECK(batch >= 1, "batch %d < 1", batch);
+    const int H = e->dims.n_audio_head, d = e->dims.n_audio_state;
+    ProfScope ps(e, WLK_KC_MISC, 4.0 * batch * H * (double)N_CTX * N_CTX * 64, 0);
+    if (type == DT_BF16X2) {
+        // split planes (the bf16x3 mode): qkv is the hi plane [batch * 1500, 3d] bf16, the lo plane right behind it;
+        // out is fp32
+        WLK_CHECK(backend == WLK_BACKEND_TCGEN05 || backend == 3, "split-plane attention runs on the tensor cores (backend 2 or 3)");
+        const bf16* hi = reinterpret_cast<const bf16*>(qkv);
+        enc_attention_tcgen05_x3(hi, hi + (size_t)batch * N_CTX * 3 * d, batch, H, d, reinterpret_cast<float*>(out), e->st);
+    } else if (backend == WLK_BACKEND_TCGEN05 || backend == 3) {
         WLK_CHECK(type == DT_BF16, "tcgen05 attention needs bf16");
-        enc_attention_tcgen05(qkv, batch, e->dims.n_audio_head, e->dims.n_audio_state, out, e->st, e->num_sms);
+        if (backend == 3) enc_attention_tcgen05_one_tile(qkv, batch, H, d, out, e->st);   // 3 = force the one-tile CTA
+        else enc_attention_tcgen05(qkv, batch, H, d, out, e->st, e->num_sms);
     } else {
-        enc_attention_simt(qkv, type, batch, e->dims.n_audio_head, e->dims.n_audio_state, out, e->st);
+        WLK_CHECK(backend == WLK_BACKEND_SIMT, "backend %d: 1 = SIMT, 2 = tcgen05, 3 = one-tile tcgen05", backend);
+        WLK_CHECK(type == DT_F32 || type == DT_BF16, "type %d: 0 = fp32, 1 = bf16, 2 = split bf16 planes", type);
+        enc_attention_simt(qkv, type, batch, H, d, out, e->st);
     }
+    WLK_API_END
+}
+
+int wlk_op_decoder_attention(wlk_engine* e, int kind, int backend, int type, int layer, const void* q, int n_jobs,
+                             const int32_t* n_rows, const int32_t* offsets, const int32_t* align_row0,
+                             const void* const* kv, float* const* align, void* out) {
+    WLK_API_BEGIN
+    LOCK(e);
+    const wlk_dims& D = e->dims;
+    const int ctx = D.n_text_ctx;
+    WLK_CHECK(kind == 0 || kind == 1, "kind %d: 0 = causal self-attention, 1 = cross-attention", kind);
+    WLK_CHECK(backend == WLK_BACKEND_SIMT || backend == WLK_BACKEND_TCGEN05, "backend %d: 1 = SIMT, 2 = tcgen05", backend);
+    WLK_CHECK(type == DT_F32 || type == DT_BF16, "type %d: 0 = fp32, 1 = bf16", type);
+    WLK_CHECK(backend == WLK_BACKEND_SIMT || type == DT_BF16, "the tcgen05 decoder attention needs bf16");
+    WLK_CHECK(layer >= 0 && layer < D.n_text_layer, "layer %d outside [0, %d)", layer, D.n_text_layer);
+    WLK_CHECK(n_jobs >= 1 && n_jobs <= 65535, "%d jobs outside [1, 65535]", n_jobs);
+    WLK_CHECK(n_rows && offsets && kv, "null argument");
+    WLK_CHECK(aligned16(q) && aligned16(out), "q and out must be non-null and 16-byte aligned");
+    const bool cross = kind == 1;
+    if (cross) WLK_CHECK(align_row0 && align, "cross-attention needs align_row0 and align");
+    std::vector<DecJob> jobs(n_jobs);
+    int R = 0, max_rows = 0;
+    for (int i = 0; i < n_jobs; ++i) {
+        const int nr = n_rows[i], off = offsets[i];
+        WLK_CHECK(nr >= 1 && off >= 0 && off <= ctx - nr, "job %d: rows at positions [%d, %d + %d) outside n_text_ctx %d",
+                  i, off, off, nr, ctx);
+        WLK_CHECK(aligned16(kv[i]), "job %d: kv must be non-null and 16-byte aligned", i);
+        DecJob& j = jobs[i];
+        memset(&j, 0, sizeof(DecJob));
+        j.row_off = R; j.n_rows = nr; j.offset = off; j.slot = i;     // slot: the job's tensor map in this call's array
+        if (cross) {
+            const int a0 = align_row0[i];
+            WLK_CHECK(a0 >= 0 && a0 <= ctx - nr, "job %d: alignment rows [%d, %d + %d) outside n_text_ctx %d", i, a0, a0, nr, ctx);
+            WLK_CHECK(aligned16(align[i]), "job %d: align must be non-null and 16-byte aligned", i);
+            j.cross_kv = kv[i]; j.align = align[i]; j.align_row0 = a0;
+        } else {
+            j.self_kv = const_cast<void*>(kv[i]);
+        }
+        R += nr;
+        max_rows = std::max(max_rows, nr);
+    }
+    const bool tc = backend == WLK_BACKEND_TCGEN05;
+    CallBuffers cb(e);
+    DecJob* jobs_dev = reinterpret_cast<DecJob*>(cb.take(jobs.size() * sizeof(DecJob)));
+    CUDA_CHECK(cudaMemcpyAsync(jobs_dev, jobs.data(), jobs.size() * sizeof(DecJob), cudaMemcpyHostToDevice, e->st));
+    uint8_t* maps_dev = nullptr;
+    if (tc) {
+        std::vector<uint8_t> maps((size_t)n_jobs * 128);
+        for (int i = 0; i < n_jobs; ++i) {
+            alignas(64) uint8_t tmap[128];
+            if (cross) make_cross_kv_tmap(tmap, kv[i], D.n_text_layer, D.n_text_head);
+            else make_self_kv_tmap(tmap, kv[i], D.n_text_layer, D.n_text_head, ctx);
+            memcpy(maps.data() + (size_t)i * 128, tmap, 128);
+        }
+        maps_dev = reinterpret_cast<uint8_t*>(cb.take(maps.size()));
+        CUDA_CHECK(cudaMemcpyAsync(maps_dev, maps.data(), maps.size(), cudaMemcpyHostToDevice, e->st));
+    }
+    ProfScope ps(e, cross ? WLK_KC_ATTN_DEC_CROSS : WLK_KC_ATTN_DEC_SELF);
+    if (cross) dec_cross_attention_layer(e, q, type, R, jobs_dev, n_jobs, max_rows, layer, maps_dev, out, tc);
+    else dec_self_attention_layer(e, q, type, R, jobs_dev, n_jobs, max_rows, layer, maps_dev, out, tc);
     WLK_API_END
 }
 

@@ -75,6 +75,9 @@ void embed_tokens(const int32_t* tokens_dev, const int32_t* pos_dev, const float
 void enc_attention_simt(const void* qkv, int type, int batch, int n_head, int d_model, void* out, cudaStream_t st);
 void enc_attention_tcgen05(const void* qkv, int batch, int n_head, int d_model, void* out, cudaStream_t st, int num_sms,
                            long long* trace_dev = nullptr);   // trace_dev: [12 tiles][8] clock64 stamps of one CTA (diagnostic)
+// always the one-query-tile CTA of attn_tc.cu (the kernel body the decoder prefills and the split-operand mode run)
+void enc_attention_tcgen05_one_tile(const void* qkv, int batch, int n_head, int d_model, void* out, cudaStream_t st,
+                                    long long* trace_dev = nullptr);
 void enc_attention_tcgen05_x3(const void* qkv_hi, const void* qkv_lo, int batch, int n_head, int d_model, float* out, cudaStream_t st);
 // fp32 -> (hi, lo) bf16 planes on the stream (gemm_tc.cu)
 void split_f32_planes_async(const float* src, bf16* hi, bf16* lo, int64_t n, cudaStream_t st);

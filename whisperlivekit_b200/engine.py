@@ -290,8 +290,24 @@ class WhisperEngine:
                                      ldc, M, N, K, int(gelu)))
 
     def op_encoder_attention(self, backend: str, qkv_ptr, dtype_code, batch, out_ptr):
-        be = {"simt": L.BACKEND_SIMT, "tcgen05": L.BACKEND_TCGEN05}[backend]
+        """dtype_code 0 = fp32, 1 = bf16, 2 = split bf16 planes (hi, lo right behind it; fp32 out)."""
+        be = {"simt": L.BACKEND_SIMT, "tcgen05": L.BACKEND_TCGEN05, "tcgen05_1tile": 3}[backend]
         L.check(self.lib.wlk_op_encoder_attention(self.h, be, qkv_ptr, dtype_code, batch, out_ptr))
+
+    def op_decoder_attention(self, kind: str, backend: str, dtype_code: int, layer: int, q_ptr, n_rows: Sequence[int],
+                             offsets: Sequence[int], kv_ptrs: Sequence[int], out_ptr,
+                             align_row0: Optional[Sequence[int]] = None, align_ptrs: Optional[Sequence[int]] = None):
+        """One decoder layer's attention (wlk_op_decoder_attention) over caller-owned caches: kind "self" (causal) or
+        "cross"; q / out packed [sum n_rows][n_text_state] by job, job i's rows at positions offsets[i] + t."""
+        k = {"self": 0, "cross": 1}[kind]
+        be = {"simt": L.BACKEND_SIMT, "tcgen05": L.BACKEND_TCGEN05}[backend]
+        n = len(n_rows)
+        nr, off = _i32(n_rows), _i32(offsets)
+        kv = (C.c_void_p * n)(*[int(p) for p in kv_ptrs])
+        a0 = _i32(align_row0) if align_row0 is not None else None
+        al = (C.c_void_p * n)(*[int(p) for p in align_ptrs]) if align_ptrs is not None else None
+        L.check(self.lib.wlk_op_decoder_attention(self.h, k, be, int(dtype_code), int(layer), q_ptr, n, _ptr(nr), _ptr(off),
+                                                  _ptr(a0) if a0 is not None else None, kv, al, out_ptr))
 
     def op_median_filter(self, x_ptr, out_ptr, rows: int, cols: int, width: int = 7) -> None:
         L.check(self.lib.wlk_op_median_filter(self.h, x_ptr, out_ptr, rows, cols, width))
